@@ -1,7 +1,12 @@
 """Benchmark of the Marigold denoising hot path (BASELINE.json metric: denoise-steps/sec @768 px).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config c2|c3|c4|c5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config c2|c3|c4|c5] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR (--impl b200) writes, after the timed work, what it computed as DIR/<name>.npy (float32): `latent`,
+the denoised latents of all members after the last timed step [E, 4, h, w], and the last end-to-end call's prediction
+(`depth` or `normals`) with, for E > 1, its `uncertainty`. Weights, image and noise are seeded, so two builds run with the
+same arguments can be compared output for output.
 
 --config selects the BASELINE.json configuration (default c2 = configs[1], the headline; the others are the
 LCM / normals / 1024-px cases of configs[2..4], same metric, members sharded round-robin over the ranks).
@@ -148,6 +153,26 @@ class ClockSampler:
                 "samples": len(sm)}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def _dump_outputs(out_dir, arrays):
+    """Save each array of `arrays` (name -> tensor or ndarray; None entries skipped) as out_dir/<name>.npy in float32."""
+    import numpy as np
+
+    arrs = {}
+    for name, a in arrays.items():
+        if a is not None:
+            a = a.detach().cpu().numpy() if hasattr(a, "detach") else a
+            arrs[name] = np.ascontiguousarray(a, dtype=np.float32)
+    total = sum(a.nbytes for a in arrs.values())
+    assert total <= DUMP_LIMIT_BYTES, f"outputs of {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte dump limit"
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, a in arrs.items():
+        np.save(d / f"{name}.npy", a)
+
+
 def _build_models(kind="full"):
     """Random-init weights of the real architecture (torch default init, seed 0): the oracle modules are only the
     weight generator here (and the checker of the cpu_baseline / --impl reference legs)."""
@@ -263,6 +288,10 @@ def run_b200(args):
     ms = parallel.barrier_max_ms(ms_local, dev)
     if B:
         assert torch.isfinite(target).all(), "non-finite latent after the timed region"
+    latent = None
+    if args.dump_outputs:                            # a collective when world > 1: every rank takes part
+        local = target if B else torch.empty(0, 4, lh, lw, device=dev)
+        latent = parallel.gather_members(local, E).cpu()
     value = E * K / (ms / 1e3)                       # member-steps of ALL ranks / max-over-ranks device time
 
     # ---- end to end through the public pipeline API: host image in, numpy map out --------------
@@ -293,6 +322,8 @@ def run_b200(args):
     h2d = img_pinned.numel() * img_pinned.element_size() + len(mine) * 4 * lh * lw * 4
     res_np = out.normals_np if cfg["task"] == "normals" else out.depth_np
     d2h = res_np.size * 4
+    if rank == 0 and args.dump_outputs:
+        _dump_outputs(args.dump_outputs, {"latent": latent, cfg["task"]: res_np, "uncertainty": out.uncertainty})
 
     # ---- dominant kernels alone (CUDA-graph replay => pure device time) ---------------------------
     kern = None
@@ -549,7 +580,12 @@ if __name__ == "__main__":
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-library-baseline", action="store_true")
     ap.add_argument("--no-kernel-roofline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed work, write what it computed as DIR/<name>.npy (float32, <= 64 MB in all)")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != "b200":
+        # the reference arm picks its resolution from a timing probe, so its outputs are not fixed by the arguments
+        ap.error("--dump-outputs needs --impl b200")
     if a.warmup < 3 and a.impl == "b200":
         a.warmup = 3
     if a.impl == "reference":
