@@ -6,312 +6,345 @@
 //   qkv : bf16 [NB * T, 3C]   (Q | K | V column blocks; head h owns columns h*64 .. h*64+63)
 //   out : bf16 [NB * T, C]
 //
-// One CTA = 128 queries of one (image, head), KV processed in blocks of 64 tokens; 192 threads:
-//   warp 0     TMA producer: Q tile (128 x 64) once, K / V tiles (64 x 64) through 3-stage rings
-//   warp 1     TMEM allocator + MMA issuer
-//                S_b = Q K_j^T          M128 N64 K64, both operands K-major, b = j & 1 (double-buffered)
-//                O  += P_b V_j          M128 N64 K64, A = P (bf16, K-major, written by the softmax warps
-//                                       into a SWIZZLE_128B smem tile), B = V in its natural [token, d]
-//                                       layout = MN-major operand (no transpose pass); O stays in TMEM
-//   warps 2-9  softmax. A query row is shared by TWO threads (warps w and w+4 own the same TMEM lane quarter):
-//                each handles 32 of the block's 64 scores, ONE TMEM read of S per block; the row max is
-//                exchanged through shared memory (named barrier per lane quarter). Halving the per-thread
-//                dependent chain and doubling the warps per scheduler is worth more than the exchange costs:
-//                the loop is bound by one warp's LDTM -> max -> exp2 -> STTM latency chain, not by a pipe.
-//                Lazy rescaling: the row keeps a reference max m_ref; P = exp2(S*c - m_ref). Only when
-//                a block's max exceeds m_ref by more than 8 (P could exceed 2^8) is O in TMEM
-//                rescaled (tcgen05.ld / st), which after the first blocks is rare; otherwise the
-//                softmax warps never wait on the PV MMA.
-// TMEM: S0 [0,64) S1 [64,128) O [128,192) -> 256 columns, two CTAs per SM (smem ~98 KB each) so the
-// exp (MUFU) phase of one CTA overlaps the load/convert/store phase of the other.
-#include <cstdlib>
+// One CTA (one per SM) = TWO 128-query tiles A and B of the same (image, head, KV split), keys in blocks of 128;
+// 320 threads:
+//   warp 0     TMA producer: Q_A and Q_B (128 x 64 each) once, K / V blocks (128 x 64) through 3-stage rings
+//   warp 1     TMEM allocator + MMA issuer, per tile t in {A, B}:
+//                S_t = Q_t K_j^T        M128 N128 K64, both operands K-major
+//                O_t += P_t V_j         M128 N64 K128, A = P_t (bf16) in TMEM (`tcgen05.mma` TS form), B = V in its
+//                                       natural [token, d] layout = MN-major operand (no transpose pass)
+//   warps 2-5  softmax of tile A, warps 6-9 softmax of tile B: one thread per query row (TMEM lane = row), 128
+//              scores per block read with four .x32 loads, row max in registers.
+// TMEM (all 512 columns, nothing aliased): S_A [0,128) S_B [128,256) P_A [256,320) P_B [320,384) O_A [384,448)
+// O_B [448,512). The issuer starts S_t(j+1) as soon as softmax t has copied S_t(j) to registers ("S drained"), so
+// while one softmax group computes exponentials the tensor core runs the other tile's QK^T or PV (ping-pong): the
+// softmax of one tile never waits for its own next S.
+// Lazy rescaling: a row keeps a reference max m_ref and P = exp2(S*c - m_ref); only when a block's max exceeds m_ref
+// by more than 8 (P could exceed 2^8) is O rescaled in TMEM, which after the first blocks of a row is rare.
+// Exponentials: kAttnPolyPairs of every 16 pairs of scores go through a degree-3 polynomial on the FMA pipe
+// (exp2_poly_f2), the rest through MUFU.EX2; the two pipes run side by side.
 #include "common.cuh"
 #include "kernels.h"
 #include "launch.h"
 
 namespace mgb {
 
-constexpr int attn_threads(int rt) { return 64 + 128 * rt; }   // producer + MMA warps, 4 RT softmax warps
-constexpr int kQBytes = 128 * 128;       // 128 rows x 64 bf16
-constexpr int kKvBytes = 64 * 128;       // 64 rows x 64 bf16
-constexpr int kPBytes = 128 * 128;       // 128 rows x 64 bf16
+constexpr int kAttnThreads = 320;
+constexpr int kTileBytes = 128 * 128;     // 128 rows x 64 bf16: a Q tile, a K block or a V block
 constexpr int kKvStages = 3;
 constexpr float kRescaleThreshold = 8.0f;  // log2 units
-constexpr int kAttnDefaultRT = 2;
-// P (bf16) goes back to tensor memory and feeds the PV MMA as a TMEM A-operand: no smem round trip and no
-// generic->async proxy fence in the softmax loop.
-// RT = softmax threads per query row (2 or 4: warps w, w+4, .. own the same TMEM lane quarter and split a block's 64
-// scores). The loop is a per-warp dependent chain (LDTM -> max -> exchange -> exp2 -> STTM), not a saturated pipe: ncu
-// reads the XU pipe (MUFU.EX2 + F2FP) at 102 %, yet converting on the integer ALU and evaluating 25-50 % of the
-// exponentials as an FMA-pipe polynomial made the kernel 7-18 % SLOWER (r01 and r02). More, shorter chains per row are
-// the lever: RT = 4 halves every thread's share and doubles the warps per scheduler.
+constexpr size_t kAttnSmemBytes = 1024 + 2 * kTileBytes + 2 * kKvStages * kTileBytes + 256;
+// Pairs of scores (out of every 16) whose exp2 is evaluated on the FMA pipe; the other pairs use MUFU.EX2. Swept on
+// B200 at T = 9216 (profiles/r03_attn_sweep.jsonl): 0 / 2 / 4 / 6 / 8 -> 162.6 / 162.6 / 158.6 / 189.0 / 183.1 us.
+constexpr int kAttnPolyPairs = 4;
+
 struct AttnParams {
-  CUtensorMap tmap_q;   // 3D {3C, T, NB}, box {64, 128, 1}
-  CUtensorMap tmap_kv;  // 3D {3C, T, NB}, box {64, 64, 1}
+  CUtensorMap tmap;   // 3D {3C, T, NB}, box {64, 128, 1}: Q tiles and K / V blocks
   bf16* out;
-  int T, C;
+  int T, C, NB;
   float scale_log2;
-  // split-KV (balances the last wave: 72 x 5 = 360 tiles on 296 CTA slots is 2 rounds of full tiles, but 1.25 rounds
-  // of quarter tiles): blockIdx.z = img * splits + split; split s covers KV blocks [s * nkv / splits, (s+1) * ...).
-  // With splits > 1 the CTA writes un-normalised fp32 O plus (m, l) per row; attn_combine_kernel merges them.
+  // split-KV: blockIdx.z = img * splits + split; split s covers KV blocks [s * nkv / splits, (s+1) * ...). With
+  // splits > 1 the CTA writes un-normalised fp32 O plus (m, l) per row; attn_combine_kernel merges them.
   int splits;
   float* part_o;    // [splits][NB][C/64][T][64]
   float* part_ml;   // [splits][NB][C/64][T][2]   (m in log2 units incl. the softmax scale, l)
 };
 
-// 64-thread named barrier of one TMEM lane quarter (constant ids: a register id makes ptxas reserve all 16)
-template <int N>
-__device__ __forceinline__ void quarter_barrier(int q) {
-  switch (q) {
-    case 0: asm volatile("bar.sync 1, %0;" ::"n"(N) : "memory"); break;
-    case 1: asm volatile("bar.sync 2, %0;" ::"n"(N) : "memory"); break;
-    case 2: asm volatile("bar.sync 3, %0;" ::"n"(N) : "memory"); break;
-    default: asm volatile("bar.sync 4, %0;" ::"n"(N) : "memory"); break;
-  }
+// exp2 of two values on the FMA pipe (no MUFU). Cody-Waite: x = j + f, j = floor(x), f in [0, 1);
+// 2^f = 1 + f (c1 + f (c2 + f c3)) (relative minimax, |rel error| <= 8.6e-5 = 2^-13.5, far below bf16's half ulp
+// 2^-9; tests/test_host.py restates it); 2^j enters as an integer add to the exponent field. floor(x) comes from
+// one round-down add of 1.5 * 2^23, whose low mantissa bits then hold j as a two's complement integer: shifted by 23
+// they are the exponent increment. x is clamped at -127 (masked keys are -inf): the result there is below 2^-126.
+constexpr float kExp2C1 = 0.6951163411140442f;
+constexpr float kExp2C2 = 0.22764700651168823f;
+constexpr float kExp2C3 = 0.07706519961357117f;
+__device__ __forceinline__ f2 f2_add_rm(f2 a, f2 b) {
+  f2 r;
+  asm("add.rm.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
+  return r;
+}
+__device__ __forceinline__ void exp2_poly_f2(float x0, float x1, float& y0, float& y1) {
+  const f2 x = f2_make(fmaxf(x0, -127.f), fmaxf(x1, -127.f));
+  const f2 t = f2_add_rm(x, f2_splat(12582912.f));             // 1.5 * 2^23 + floor(x)
+  const f2 f = f2_sub(x, f2_sub(t, f2_splat(12582912.f)));
+  f2 q = f2_fma(f2_splat(kExp2C3), f, f2_splat(kExp2C2));
+  q = f2_fma(q, f, f2_splat(kExp2C1));
+  q = f2_fma(q, f, f2_splat(1.f));
+  float q0, q1, t0, t1;
+  f2_split(q, q0, q1);
+  f2_split(t, t0, t1);
+  y0 = __uint_as_float(__float_as_uint(q0) + (__float_as_uint(t0) << 23));
+  y1 = __uint_as_float(__float_as_uint(q1) + (__float_as_uint(t1) << 23));
 }
 
-template <int RT>
-__global__ void __launch_bounds__(attn_threads(RT), 2) flash_attn64_kernel(const __grid_constant__ AttnParams p) {
+// base + off, computed where it is used: keeps ptxas from hoisting every TMEM column address of the softmax loop into
+// its own register for the whole loop (the 128 scores of a row already take most of the 168 available)
+__device__ __forceinline__ uint32_t addr_at_use(uint32_t base, uint32_t off) {
+  uint32_t r;
+  asm volatile("add.u32 %0, %1, %2;" : "=r"(r) : "r"(base), "r"(off));
+  return r;
+}
+
+__global__ void __launch_bounds__(kAttnThreads, 1) flash_attn64_kernel(const __grid_constant__ AttnParams p) {
   pdl_launch_dependents();
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* sQ = smem;
-  uint8_t* sK = sQ + kQBytes;
-  uint8_t* sV = sK + kKvStages * kKvBytes;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(sV + kKvStages * kKvBytes);
+  uint8_t* sQ = smem;                        // [2] A, B
+  uint8_t* sK = sQ + 2 * kTileBytes;         // [kKvStages]
+  uint8_t* sV = sK + kKvStages * kTileBytes; // [kKvStages]
+  uint64_t* bars = reinterpret_cast<uint64_t*>(sV + kKvStages * kTileBytes);
   uint64_t* q_full = bars;                   // 1
   uint64_t* k_full = bars + 1;               // [3]
   uint64_t* k_empty = bars + 4;              // [3]
   uint64_t* v_full = bars + 7;               // [3]
   uint64_t* v_empty = bars + 10;             // [3]
-  uint64_t* s_full = bars + 13;              // [2]
-  uint64_t* p_full = bars + 15;              // [2]  (128 arrivals)
-  uint64_t* p_empty = bars + 17;             // [2]  PV(j) complete: P buffer free, O updated
-  uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(bars + 19);
-  float* s_xch = reinterpret_cast<float*>(bars + 20);   // [2 slots][4 quarters][2 halves][32 lanes] row-max exchange (+ final l)
+  uint64_t* s_full = bars + 13;              // [2 tiles]  S_t(j) computed
+  uint64_t* s_drained = bars + 15;           // [2]  (128 arrivals) S_t(j) copied to registers: S_t may be rewritten
+  uint64_t* p_full = bars + 17;              // [2]  (128 arrivals) P_t(j) stored (and O_t rescaled)
+  uint64_t* pv_done = bars + 19;             // [2]  PV_t(j) complete: P_t free, O_t updated
+  uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(bars + 21);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int q0 = blockIdx.x * 128, head = blockIdx.y, img = blockIdx.z / p.splits, split = blockIdx.z % p.splits;
-  const int nkv_all = (p.T + 63) / 64;
+  const int q0 = blockIdx.x * 256, head = blockIdx.y, img = blockIdx.z / p.splits, split = blockIdx.z % p.splits;
+  const bool has_b = q0 + 128 < p.T;         // the B tile of the last pair may be empty
+  const int nkv_all = (p.T + 127) / 128;
   const int jb0 = split * nkv_all / p.splits;                 // first KV block of this CTA
   const int nkv = (split + 1) * nkv_all / p.splits - jb0;     // its number of KV blocks (>= 1: host keeps splits <= nkv_all)
 
   if (warp == 0 && lane == 0) {
-    tma_prefetch_desc(&p.tmap_q);
-    tma_prefetch_desc(&p.tmap_kv);
+    tma_prefetch_desc(&p.tmap);
     mbar_init(q_full, 1);
     for (int s = 0; s < kKvStages; ++s) {
       mbar_init(&k_full[s], 1); mbar_init(&k_empty[s], 1);
       mbar_init(&v_full[s], 1); mbar_init(&v_empty[s], 1);
     }
-    for (int b = 0; b < 2; ++b) {
-      mbar_init(&s_full[b], 1);
-      mbar_init(&p_full[b], 128 * RT);
-      mbar_init(&p_empty[b], 1);
+    for (int t = 0; t < 2; ++t) {
+      mbar_init(&s_full[t], 1);
+      mbar_init(&s_drained[t], 128);
+      mbar_init(&p_full[t], 128);
+      mbar_init(&pv_done[t], 1);
     }
     fence_mbar_init();
   }
   if (warp == 1) {
-    tmem_alloc(tmem_ptr_smem, 256);
+    tmem_alloc(tmem_ptr_smem, 512);
     tmem_relinquish();
   }
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr_smem;
-  const uint32_t tmem_o = tmem_base + 128;
   pdl_wait();
 
   // Producer and MMA issuer are single-thread latency chains (see gemm_tc.cu): whole loop inside one elected
-  // thread, shared-window addresses and descriptor words precomputed, counters instead of % and /. The first
-  // version (elect + warp sync + generic addressing per phase) took ~1300 cycles per KV block and bounded the
-  // whole kernel (384k cycles for T = 9216 = 2 waves x 144 blocks x 1333).
+  // thread, shared-window addresses and descriptor words precomputed, counters instead of % and /.
   if (warp == 0) {
     // ===================== TMA producer =====================
     if (elect_one()) {
       const uint32_t kfull = smem_u32(k_full), kempty = smem_u32(k_empty), vfull = smem_u32(v_full),
                      vempty = smem_u32(v_empty);
       const uint32_t sK_a = smem_u32(sK), sV_a = smem_u32(sV);
-      mbar_arrive_expect_tx(q_full, kQBytes);
-      tma_load_3d(sQ, &p.tmap_q, q_full, head * 64, q0, img);
+      mbar_arrive_expect_tx(q_full, has_b ? 2 * kTileBytes : kTileBytes);
+      tma_load_3d(sQ, &p.tmap, q_full, head * 64, q0, img);
+      if (has_b) tma_load_3d(sQ + kTileBytes, &p.tmap, q_full, head * 64, q0 + 128, img);
       const int ck = p.C + head * 64, cv = 2 * p.C + head * 64;
       uint32_t s = 0, ph = 0;
       for (int j = 0; j < nkv; ++j) {
         mbar_wait_a(kempty + s * 8, ph ^ 1);
-        mbar_expect_tx_a(kfull + s * 8, kKvBytes);
-        tma_load_3d_a(sK_a + s * kKvBytes, &p.tmap_kv, kfull + s * 8, ck, (jb0 + j) * 64, img);
+        mbar_expect_tx_a(kfull + s * 8, kTileBytes);
+        tma_load_3d_a(sK_a + s * kTileBytes, &p.tmap, kfull + s * 8, ck, (jb0 + j) * 128, img);
         mbar_wait_a(vempty + s * 8, ph ^ 1);
-        mbar_expect_tx_a(vfull + s * 8, kKvBytes);
-        tma_load_3d_a(sV_a + s * kKvBytes, &p.tmap_kv, vfull + s * 8, cv, (jb0 + j) * 64, img);
+        mbar_expect_tx_a(vfull + s * 8, kTileBytes);
+        tma_load_3d_a(sV_a + s * kTileBytes, &p.tmap, vfull + s * 8, cv, (jb0 + j) * 128, img);
         if (++s == kKvStages) { s = 0; ph ^= 1; }
       }
     }
   } else if (warp == 1) {
     // ===================== MMA issuer =====================
     if (elect_one()) {
-      constexpr uint32_t idesc_s = umma_idesc_bf16(128, 64, false);
+      constexpr uint32_t idesc_s = umma_idesc_bf16(128, 128, false);
       constexpr uint32_t idesc_pv = umma_idesc_bf16(128, 64, true);
       constexpr uint32_t kHi = uint32_t(kDescSw128Hi >> 32), kLbo = 1u << 16;
       const uint32_t kfull = smem_u32(k_full), kempty = smem_u32(k_empty), vfull = smem_u32(v_full),
-                     vempty = smem_u32(v_empty), sfull = smem_u32(s_full), pfull = smem_u32(p_full),
-                     pempty = smem_u32(p_empty);
-      const uint32_t dq_lo = (smem_u32(sQ) >> 4) | kLbo, dk_lo0 = (smem_u32(sK) >> 4) | kLbo,
+                     vempty = smem_u32(v_empty), sfull = smem_u32(s_full), sdrained = smem_u32(s_drained),
+                     pfull = smem_u32(p_full), pvdone = smem_u32(pv_done);
+      const uint32_t dq_lo0 = (smem_u32(sQ) >> 4) | kLbo, dk_lo0 = (smem_u32(sK) >> 4) | kLbo,
                      dv_lo0 = (smem_u32(sV) >> 4) | kLbo;
-      uint32_t ks = 0, kph = 0, vs = 0, vph = 0;
-      auto issue_s = [&](int j) {
-        mbar_wait_a(kfull + ks * 8, kph);
-        const uint32_t dk_lo = dk_lo0 + ks * uint32_t(kKvBytes >> 4);
-        const uint32_t ts = tmem_base + uint32_t(j & 1) * 64;
-        umma_bf16(ts, make_u64(dq_lo, kHi), make_u64(dk_lo, kHi), idesc_s, 0u);
-        umma_bf16(ts, make_u64(dq_lo + 2, kHi), make_u64(dk_lo + 2, kHi), idesc_s, 1u);
-        umma_bf16(ts, make_u64(dq_lo + 4, kHi), make_u64(dk_lo + 4, kHi), idesc_s, 1u);
-        umma_bf16(ts, make_u64(dq_lo + 6, kHi), make_u64(dk_lo + 6, kHi), idesc_s, 1u);
-        umma_commit_a(kempty + ks * 8);
-        umma_commit_a(sfull + uint32_t(j & 1) * 8);
-        if (++ks == kKvStages) { ks = 0; kph ^= 1; }
+      const int ntiles = has_b ? 2 : 1;
+      // S_t = Q_t K^T into TMEM columns [128 t, 128 t + 128): 4 x K=16 (32 B steps inside the 128 B swizzled rows)
+      auto issue_s = [&](int t, uint32_t ks) {
+        const uint32_t dq_lo = dq_lo0 + uint32_t(t) * uint32_t(kTileBytes >> 4);
+        const uint32_t dk_lo = dk_lo0 + ks * uint32_t(kTileBytes >> 4);
+        const uint32_t ts = tmem_base + uint32_t(t) * 128;
+#pragma unroll
+        for (int k = 0; k < 4; ++k)
+          umma_bf16(ts, make_u64(dq_lo + 2 * k, kHi), make_u64(dk_lo + 2 * k, kHi), idesc_s, k > 0 ? 1u : 0u);
+        umma_commit_a(sfull + uint32_t(t) * 8);
       };
+      // O_t += P_t V: A = P_t (bf16) in TMEM, 16 keys = 8 columns per K=16 step; B = V [kv, d] d-contiguous
+      // (MN-major): 16 kv rows = 2048 B per step
+      auto issue_pv = [&](int t, uint32_t vs, bool acc) {
+        const uint32_t tp = tmem_base + 256 + uint32_t(t) * 64, to = tmem_base + 384 + uint32_t(t) * 64;
+        const uint32_t dv_lo = dv_lo0 + vs * uint32_t(kTileBytes >> 4);
+#pragma unroll
+        for (int k = 0; k < 8; ++k)
+          umma_bf16_ts(to, tp + 8 * k, make_u64(dv_lo + 128 * k, kHi), idesc_pv, (acc || k > 0) ? 1u : 0u);
+        umma_commit_a(pvdone + uint32_t(t) * 8);
+      };
+      uint32_t ks = 0, kph = 0, vs = 0, vph = 0;
       mbar_wait_a(smem_u32(q_full), 0);
-      issue_s(0);
+      mbar_wait_a(kfull, 0);
+      tc_fence_after();
+      for (int t = 0; t < ntiles; ++t) issue_s(t, 0);
+      umma_commit_a(kempty);
+      ks = 1;
       for (int j = 0; j < nkv; ++j) {
-        // S(j+1) goes into the other S buffer: free because softmax(j-1) signalled p_full(j-1), which
-        // this thread waited for before PV(j-1)
-        if (j + 1 < nkv) issue_s(j + 1);
-        const uint32_t b = uint32_t(j & 1);
-        mbar_wait_a(pfull + b * 8, uint32_t(j >> 1) & 1u);
+        const uint32_t ph = uint32_t(j) & 1u;
+        const bool next = j + 1 < nkv;
+        if (next) mbar_wait_a(kfull + ks * 8, kph);
         mbar_wait_a(vfull + vs * 8, vph);
-        tc_fence_after();
-        // A: P (bf16) in TMEM, 16 bf16 = 8 columns per K=16 step; B: V [kv, d] d-contiguous (MN-major):
-        // 16 kv rows = 2048 B per K=16 step
-        const uint32_t tp = tmem_base + 192 + b * 32;
-        const uint32_t dv_lo = dv_lo0 + vs * uint32_t(kKvBytes >> 4);
-        umma_bf16_ts(tmem_o, tp, make_u64(dv_lo, kHi), idesc_pv, j > 0 ? 1u : 0u);
-        umma_bf16_ts(tmem_o, tp + 8, make_u64(dv_lo + 128, kHi), idesc_pv, 1u);
-        umma_bf16_ts(tmem_o, tp + 16, make_u64(dv_lo + 256, kHi), idesc_pv, 1u);
-        umma_bf16_ts(tmem_o, tp + 24, make_u64(dv_lo + 384, kHi), idesc_pv, 1u);
+        for (int t = 0; t < ntiles; ++t) {
+          if (next) {   // S_t(j+1) as soon as softmax t holds S_t(j) in registers
+            mbar_wait_a(sdrained + uint32_t(t) * 8, ph);
+            tc_fence_after();
+            issue_s(t, ks);
+          }
+          mbar_wait_a(pfull + uint32_t(t) * 8, ph);
+          tc_fence_after();
+          issue_pv(t, vs, j > 0);
+        }
+        if (next) {
+          umma_commit_a(kempty + ks * 8);
+          if (++ks == kKvStages) { ks = 0; kph ^= 1; }
+        }
         umma_commit_a(vempty + vs * 8);
-        umma_commit_a(pempty + b * 8);
         if (++vs == kKvStages) { vs = 0; vph ^= 1; }
       }
     }
     __syncwarp();
-  } else {
-    // ===================== softmax =====================
-    constexpr int NS = 64 / RT;             // scores (and O columns) per thread
-    const int q = warp & 3;                 // TMEM lane quarter
-    const int h = (warp - 2) >> 2;          // which part of the block's 64 scores / of O's 64 columns
-    const int row = q * 32 + lane;
-    const uint32_t lane_off = uint32_t(q * 32) << 16;
+  } else if (warp < 6 || has_b) {
+    // ===================== softmax (tile t) =====================
+    const int t = warp >= 6 ? 1 : 0;
+    const int qw = warp & 3;                 // TMEM lane quarter
+    const int row = qw * 32 + lane;
+    const uint32_t lane_off = uint32_t(qw * 32) << 16;
+    const uint32_t tS = tmem_base + lane_off + uint32_t(t) * 128, tP = tmem_base + lane_off + 256 + uint32_t(t) * 64,
+                   tO = tmem_base + lane_off + 384 + uint32_t(t) * 64;
     float m_ref = 0.f, l_run = 0.f;
     for (int j = 0; j < nkv; ++j) {
-      const int b = j & 1, u = j >> 1;
-      mbar_wait(&s_full[b], u & 1);
+      const uint32_t ph = uint32_t(j) & 1u;
+      mbar_wait(&s_full[t], ph);
       tc_fence_after();
-      uint32_t r[NS];
-      TmemIO<NS>::ld(tmem_base + lane_off + b * 64 + h * NS, r);
+      uint32_t r[128];
+      tmem_ld32(tS, *reinterpret_cast<uint32_t(*)[32]>(r));
+      tmem_ld32(addr_at_use(tS, 32), *reinterpret_cast<uint32_t(*)[32]>(r + 32));
+      tmem_ld32(addr_at_use(tS, 64), *reinterpret_cast<uint32_t(*)[32]>(r + 64));
+      tmem_ld32(addr_at_use(tS, 96), *reinterpret_cast<uint32_t(*)[32]>(r + 96));
       tmem_wait_ld();
-      const int kv_valid = p.T - (jb0 + j) * 64 - h * NS;   // >= NS except possibly in the last block
-      if (kv_valid < NS) {                          // ragged tail (T % 64 != 0): mask once, then share the fast path
+      tc_fence_before();
+      mbar_arrive(&s_drained[t]);
+      const int kv_valid = p.T - (jb0 + j) * 128;   // >= 128 except possibly in the last block
+      if (kv_valid < 128) {                         // ragged tail: mask once, then share the fast path
 #pragma unroll
-        for (int i = 0; i < NS; ++i)
+        for (int i = 0; i < 128; ++i)
           if (i >= kv_valid) r[i] = 0xff800000u;    // -inf
       }
-      // partial row max with 4 independent chains, then the exchange with the warps owning the other scores of the row
-      float mxa = __uint_as_float(r[0]), mxb = __uint_as_float(r[1]), mxc = __uint_as_float(r[2]),
-            mxd = __uint_as_float(r[3]);
+      // row max with 4 independent chains
+      float mx[4];
 #pragma unroll
-      for (int i = 4; i < NS; i += 4) {
-        mxa = fmaxf(mxa, __uint_as_float(r[i]));
-        mxb = fmaxf(mxb, __uint_as_float(r[i + 1]));
-        mxc = fmaxf(mxc, __uint_as_float(r[i + 2]));
-        mxd = fmaxf(mxd, __uint_as_float(r[i + 3]));
-      }
-      float mx = fmaxf(fmaxf(mxa, mxb), fmaxf(mxc, mxd));
-      float* xs = s_xch + ((b * 4 + q) * RT) * 32;
-      xs[h * 32 + lane] = mx;
-      quarter_barrier<32 * RT>(q);
+      for (int c = 0; c < 4; ++c) mx[c] = __uint_as_float(r[c]);
 #pragma unroll
-      for (int k = 1; k < RT; ++k) mx = fmaxf(mx, xs[((h + k) % RT) * 32 + lane]);
-      const float m_blk = mx * p.scale_log2;
+      for (int i = 4; i < 128; i += 4)
+#pragma unroll
+        for (int c = 0; c < 4; ++c) mx[c] = fmaxf(mx[c], __uint_as_float(r[i + c]));
+      const float m_blk = fmaxf(fmaxf(mx[0], mx[1]), fmaxf(mx[2], mx[3])) * p.scale_log2;
+      // Lazy rescaling: the O rescale itself runs after the P stores, when the scores no longer hold registers
+      bool rescale = false;
+      float alpha = 1.f;
       if (j == 0) {
         m_ref = m_blk;
       } else {
+        // P_t and O_t are free once PV_t(j-1) has completed
+        mbar_wait(&pv_done[t], ph ^ 1);
+        tc_fence_after();
         const bool need = m_blk > m_ref + kRescaleThreshold;
-        if (__any_sync(0xffffffffu, need)) {      // identical decision in every warp of the quarter
-          // rescale O (and l) of the rows that need it; other rows multiply by 1
-          const float m_new = need ? m_blk : m_ref;
-          const float alpha = ex2_approx(m_ref - m_new);
-          m_ref = m_new;
+        rescale = __any_sync(0xffffffffu, need);    // the TMEM loads of O are warp-collective
+        if (need) {                                 // other rows of the warp multiply O by 1
+          alpha = ex2_approx(m_ref - m_blk);
+          m_ref = m_blk;
           l_run *= alpha;
-          mbar_wait(&p_empty[(j - 1) & 1], ((j - 1) >> 1) & 1);   // every PV issued so far has completed
-          tc_fence_after();
-          uint32_t o[NS];
-          TmemIO<NS>::ld(tmem_o + lane_off + h * NS, o);
-          tmem_wait_ld();
-#pragma unroll
-          for (int i = 0; i < NS; ++i) o[i] = __float_as_uint(__uint_as_float(o[i]) * alpha);
-          TmemIO<NS>::st(tmem_o + lane_off + h * NS, o);
-          tmem_wait_st();
         }
       }
-      // P = exp2(S * c - m_ref) (exp2(-inf) = 0 masks the tail); bf16 pairs; 4 partial row sums
-      // (the scale-and-shift and the row sums go through FFMA2 / FADD2: two scores per instruction)
-      uint32_t pk[NS / 2];
-      f2 ls01 = f2_splat(0.f), ls23 = ls01;
+      // P = exp2(S * c - m_ref) (exp2(-inf) = 0 masks the tail); bf16 pairs; packed partial row sums.
+      // Per 32 scores: the scale-and-shift (FFMA2), exponentials (kAttnPolyPairs of 16 pairs on the FMA pipe), F2FP packs,
+      // row sums (FADD2), one 16-column store of P.
       const f2 sc2 = f2_splat(p.scale_log2), nm2 = f2_splat(-m_ref);
+      f2 ls0 = f2_splat(0.f), ls1 = ls0;
 #pragma unroll
-      for (int i = 0; i < NS / 4; ++i) {
-        float t0, t1, t2, t3;
-        f2_split(f2_fma(f2_make(__uint_as_float(r[4 * i]), __uint_as_float(r[4 * i + 1])), sc2, nm2), t0, t1);
-        f2_split(f2_fma(f2_make(__uint_as_float(r[4 * i + 2]), __uint_as_float(r[4 * i + 3])), sc2, nm2), t2, t3);
-        const float a0 = ex2_approx(t0), a1 = ex2_approx(t1), a2 = ex2_approx(t2), a3 = ex2_approx(t3);
-        ls01 = f2_add(ls01, f2_make(a0, a1));
-        ls23 = f2_add(ls23, f2_make(a2, a3));
-        pk[2 * i] = pack_bf16x2(a0, a1);
-        pk[2 * i + 1] = pack_bf16x2(a2, a3);
+      for (int c = 0; c < 4; ++c) {
+        uint32_t pk[16];
+#pragma unroll
+        for (int i = 0; i < 16; ++i) {
+          float t0, t1, a0, a1;
+          f2_split(f2_fma(f2_make(__uint_as_float(r[32 * c + 2 * i]), __uint_as_float(r[32 * c + 2 * i + 1])), sc2, nm2),
+                   t0, t1);
+          if (((i + 1) * kAttnPolyPairs) / 16 != (i * kAttnPolyPairs) / 16) {   // spread evenly over the 16 pairs
+            exp2_poly_f2(t0, t1, a0, a1);
+          } else {
+            a0 = ex2_approx(t0);
+            a1 = ex2_approx(t1);
+          }
+          if (i & 1) ls1 = f2_add(ls1, f2_make(a0, a1));
+          else ls0 = f2_add(ls0, f2_make(a0, a1));
+          pk[i] = pack_bf16x2(a0, a1);
+        }
+        tmem_st16(addr_at_use(tP, c * 16), pk);
       }
       {
-        float ls0, ls1, ls2, ls3;
-        f2_split(ls01, ls0, ls1);
-        f2_split(ls23, ls2, ls3);
-        l_run += (ls0 + ls1) + (ls2 + ls3);
+        float s0, s1, s2, s3;
+        f2_split(ls0, s0, s1);
+        f2_split(ls1, s2, s3);
+        l_run += (s0 + s1) + (s2 + s3);
       }
-      // P buffer b was last read by PV(j-2)
-      mbar_wait(&p_empty[b], (u & 1) ^ 1);
-      TmemIO<NS / 2>::st(tmem_base + 192 + b * 32 + h * (NS / 2) + lane_off, pk);
+      if (rescale) {
+#pragma unroll
+        for (int h = 0; h < 2; ++h) {
+          uint32_t o[32];
+          tmem_ld32(addr_at_use(tO, h * 32), o);
+          tmem_wait_ld();
+#pragma unroll
+          for (int i = 0; i < 32; ++i) o[i] = __float_as_uint(__uint_as_float(o[i]) * alpha);
+          tmem_st32(addr_at_use(tO, h * 32), o);
+        }
+      }
       tmem_wait_st();
       tc_fence_before();
-      mbar_arrive(&p_full[b]);
+      mbar_arrive(&p_full[t]);
     }
-    // epilogue: O / l. The parts of a row add their partial sums through the exchange buffer
-    // (slot (nkv & 1): not the one the last block's max exchange used).
-    float* xl = s_xch + (((nkv & 1) * 4 + q) * RT) * 32;
-    xl[h * 32 + lane] = l_run;
-    quarter_barrier<32 * RT>(q);
-    float l_tot = 0.f;
-#pragma unroll
-    for (int k = 0; k < RT; ++k) l_tot += xl[k * 32 + lane];      // same order in every part: identical l_tot
-    mbar_wait(&p_empty[(nkv - 1) & 1], ((nkv - 1) >> 1) & 1);
+    // epilogue: O / l, or the un-normalised split partial
+    mbar_wait(&pv_done[t], uint32_t(nkv - 1) & 1u);
     tc_fence_after();
-    const int qrow = q0 + row;
-    uint32_t o0[NS];
-    TmemIO<NS>::ld(tmem_o + lane_off + h * NS, o0);
+    const int qrow = q0 + t * 128 + row;
+    uint32_t o[64];
+    tmem_ld32(tO, *reinterpret_cast<uint32_t(*)[32]>(o));
+    tmem_ld32(tO + 32, *reinterpret_cast<uint32_t(*)[32]>(o + 32));
     tmem_wait_ld();
     if (qrow < p.T) {
       if (p.splits == 1) {
-        const float inv = 1.f / l_tot;
-        uint4* dst = reinterpret_cast<uint4*>(p.out + ((size_t)img * p.T + qrow) * p.C + head * 64 + h * NS);
+        const float inv = 1.f / l_run;
+        uint4* dst = reinterpret_cast<uint4*>(p.out + ((size_t)img * p.T + qrow) * p.C + head * 64);
 #pragma unroll
-        for (int i = 0; i < NS / 8; ++i)
-          dst[i] = make_uint4(pack_bf16x2(__uint_as_float(o0[8 * i]) * inv, __uint_as_float(o0[8 * i + 1]) * inv),
-                              pack_bf16x2(__uint_as_float(o0[8 * i + 2]) * inv, __uint_as_float(o0[8 * i + 3]) * inv),
-                              pack_bf16x2(__uint_as_float(o0[8 * i + 4]) * inv, __uint_as_float(o0[8 * i + 5]) * inv),
-                              pack_bf16x2(__uint_as_float(o0[8 * i + 6]) * inv, __uint_as_float(o0[8 * i + 7]) * inv));
+        for (int i = 0; i < 8; ++i)
+          dst[i] = make_uint4(pack_bf16x2(__uint_as_float(o[8 * i]) * inv, __uint_as_float(o[8 * i + 1]) * inv),
+                              pack_bf16x2(__uint_as_float(o[8 * i + 2]) * inv, __uint_as_float(o[8 * i + 3]) * inv),
+                              pack_bf16x2(__uint_as_float(o[8 * i + 4]) * inv, __uint_as_float(o[8 * i + 5]) * inv),
+                              pack_bf16x2(__uint_as_float(o[8 * i + 6]) * inv, __uint_as_float(o[8 * i + 7]) * inv));
       } else {
-        const size_t prow = ((size_t(split) * gridDim.z / p.splits + img) * gridDim.y + head) * p.T + qrow;
-        uint4* dst = reinterpret_cast<uint4*>(p.part_o + prow * 64 + h * NS);
+        const size_t prow = ((size_t(split) * p.NB + img) * gridDim.y + head) * p.T + qrow;
+        uint4* dst = reinterpret_cast<uint4*>(p.part_o + prow * 64);
 #pragma unroll
-        for (int i = 0; i < NS / 4; ++i) dst[i] = make_uint4(o0[4 * i], o0[4 * i + 1], o0[4 * i + 2], o0[4 * i + 3]);
-        if (h == 0) *reinterpret_cast<float2*>(p.part_ml + prow * 2) = make_float2(m_ref, l_tot);
+        for (int i = 0; i < 16; ++i) dst[i] = make_uint4(o[4 * i], o[4 * i + 1], o[4 * i + 2], o[4 * i + 3]);
+        *reinterpret_cast<float2*>(p.part_ml + prow * 2) = make_float2(m_ref, l_run);
       }
     }
     tc_fence_before();
@@ -319,7 +352,7 @@ __global__ void __launch_bounds__(attn_threads(RT), 2) flash_attn64_kernel(const
   __syncthreads();
   if (warp == 1) {
     tc_fence_after();
-    tmem_dealloc(tmem_base, 256);
+    tmem_dealloc(tmem_base, 512);
   }
 }
 
@@ -354,17 +387,21 @@ __global__ void __launch_bounds__(256) attn_combine_kernel(const float* __restri
                     pack_bf16x2(acc[4] * inv, acc[5] * inv), pack_bf16x2(acc[6] * inv, acc[7] * inv));
 }
 
-// KV splits that minimise the number of CTA rounds (2 CTAs per SM) weighted by the split's length
+// KV splits that minimise the number of CTA rounds (one CTA per SM, one CTA = a pair of 128-query tiles) weighted by
+// the split's length in 128-key blocks plus a per-CTA fixed cost (prologue, Q load, first S, epilogue) and the
+// combine pass. Both costs fitted to forced split counts 1..6 at T = 9216, NB = 1 on B200 (182-242 us,
+// profiles/r03_attn_sweep.jsonl): 1.5 us per block and round, fixed cost 4 blocks, combine 11 blocks. The same model
+// keeps NB = 8 unsplit (measured: 1216 us unsplit, 1345-1579 us with 2-6 splits).
+constexpr double kAttnCtaFixedBlocks = 4.0;
+constexpr double kAttnCombineBlocks = 11.0;
 int flash_attn64_splits(int NB, int T, int C) {
-  const int units = ((T + 127) / 128) * (C / 64) * NB, nkv = (T + 63) / 64, slots = 148 * 2;
+  const int units = ((T + 255) / 256) * (C / 64) * NB, nkv = (T + 127) / 128, slots = 148;
   int best = 1;
   double best_t = 1e30;
   for (int s = 1; s <= 8; ++s) {
-    if (s > 1 && nkv / s < 6) break;
+    if (s > 1 && nkv / s < 3) break;
     const double rounds = double((units * s + slots - 1) / slots);
-    // measured (r01, T = 9216): a CTA's fixed cost (prologue, Q load, first S, epilogue) is worth ~15 KV blocks,
-    // the combine pass ~8
-    const double t = rounds * (double(nkv) / s + 15.0) + (s > 1 ? 8.0 : 0.0);
+    const double t = rounds * (double(nkv) / s + kAttnCtaFixedBlocks) + (s > 1 ? kAttnCombineBlocks : 0.0);
     if (t < best_t - 1e-9) { best_t = t; best = s; }
   }
   return best;
@@ -384,12 +421,10 @@ int launch_flash_attn64(const bf16* qkv, bf16* out, int NB, int T, int C, float 
   AttnParams p;
   const uint64_t dims[3] = {uint64_t(3 * C), uint64_t(T), uint64_t(NB)};
   const uint64_t strides[2] = {uint64_t(3 * C) * 2, uint64_t(T) * 3 * C * 2};
-  const uint32_t box_q[3] = {64, 128, 1}, box_kv[3] = {64, 64, 1};
-  int rc = make_tmap_3d(&p.tmap_q, qkv, dims, strides, box_q);
+  const uint32_t box[3] = {64, 128, 1};
+  int rc = make_tmap_3d(&p.tmap, qkv, dims, strides, box);
   if (rc) return rc;
-  rc = make_tmap_3d(&p.tmap_kv, qkv, dims, strides, box_kv);
-  if (rc) return rc;
-  p.out = out; p.T = T; p.C = C;
+  p.out = out; p.T = T; p.C = C; p.NB = NB;
   p.scale_log2 = scale * 1.4426950408889634f;
   p.splits = 1; p.part_o = nullptr; p.part_ml = nullptr;
   {
@@ -400,19 +435,15 @@ int launch_flash_attn64(const bf16* qkv, bf16* out, int NB, int T, int C, float 
       p.part_ml = ws + size_t(sp) * NB * (C / 64) * T * 64;
     }
   }
-  static const size_t dbg_pad = getenv("MGB_ATTN_SMEM_PAD") ? size_t(atoi(getenv("MGB_ATTN_SMEM_PAD"))) : 0;   // debug: force 1 CTA/SM
-  const size_t smem = 1024 + kQBytes + 2 * kKvStages * kKvBytes + 256 + 4096 + dbg_pad;
-  // softmax threads per row: MGB_ATTN_RT = 2 | 4
-  static const int rt = getenv("MGB_ATTN_RT") ? atoi(getenv("MGB_ATTN_RT")) : kAttnDefaultRT;
-  void (*kern)(AttnParams) = rt == 4 ? flash_attn64_kernel<4> : flash_attn64_kernel<2>;
   static bool attr_set = false;
   if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
+    cudaError_t e = cudaFuncSetAttribute(flash_attn64_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         int(kAttnSmemBytes));
     if (e != cudaSuccess) { set_error("flash_attn64 attr: %s", cudaGetErrorString(e)); return MGB_ERR_CUDA; }
     attr_set = true;
   }
-  dim3 grid((T + 127) / 128, C / 64, NB * p.splits);
-  cudaError_t e = launch_k(kern, grid, attn_threads(rt == 4 ? 4 : 2), smem, stream, p);
+  const dim3 grid((T + 255) / 256, C / 64, NB * p.splits);
+  cudaError_t e = launch_k(flash_attn64_kernel, grid, kAttnThreads, kAttnSmemBytes, stream, p);
   if (e == cudaSuccess) e = cudaGetLastError();
   if (e != cudaSuccess) { set_error("flash_attn64 launch: %s", cudaGetErrorString(e)); return MGB_ERR_CUDA; }
   if (p.splits > 1) {
