@@ -165,13 +165,32 @@ int mgb_resize(const void* src_dev, int32_t src_is_u8, int32_t NC, int32_t H, in
  * out_hwc_dev uint8 [HW,3]; lut_dev uint8 [256,3] = the colour map's 256-entry table * 255, truncated. */
 int mgb_colorize(const float* depth_dev, int64_t HW, float dmin, float dmax, const uint8_t* lut_dev, uint8_t* out_hwc_dev,
                  void* stream);
+/* Scratch of every mgb_eval_* call: a fixed size, independent of the image. */
+size_t mgb_eval_ws_bytes(void);
 /* Least-squares scale / shift alignment to the ground truth over the valid pixels (src/util/alignment.py:35-82), the
  * clips of script/depth/eval.py:201-207 and the masked depth metrics of src/util/metric.py:64-191 in two passes and ONE
- * synchronisation. mask_dev uint8 [HW] or NULL; aligned_out_dev fp32 [HW] or NULL; ws_dev: mgb_eval_ws_bytes() bytes.
- * out_host[13] = {scale, shift, n_valid, abs_rel, sq_rel, rmse, rmse_log, log10, delta1, delta2, delta3, i_rmse, silog}. */
-size_t mgb_eval_ws_bytes(void);
-int mgb_eval_depth(const float* pred_dev, const float* gt_dev, const uint8_t* mask_dev, int64_t HW, int32_t least_squares,
+ * synchronisation. alignment: 0 none, 1 least squares in depth ("least_square"), 2 least squares in disparity
+ * ("least_square_disparity", eval.py:179-199 with depth2disparity, alignment.py:85-95: fit pred to 1 / gt over
+ * mask & gt > 0 & pred > 0, depth = 1 / clip(pred * scale + shift, 1e-3)). mask_dev uint8 [HW] or NULL; aligned_out_dev
+ * fp32 [HW] or NULL (the final clipped depth); ws_dev: mgb_eval_ws_bytes() bytes.
+ * out_host[13] = {scale, shift, n_valid, abs_rel, sq_rel, rmse, rmse_log, log10, delta1, delta2, delta3, i_rmse, silog}
+ * (scale, shift in disparity space for alignment 2). */
+int mgb_eval_depth(const float* pred_dev, const float* gt_dev, const uint8_t* mask_dev, int64_t HW, int32_t alignment,
                    float dmin, float dmax, float* aligned_out_dev, void* ws_dev, double* out_host, void* stream);
+/* compute_cosine_error(masked=True) and the normals metrics mean / median / rmse / sub5 .. sub30_error
+ * (src/util/metric.py:194-257 as script/normals/eval.py:145-157 calls them) with ONE synchronisation; the median is an
+ * exact order statistic on the device (the reference copies the error map to the host for np.median).
+ * pred_dev, gt_dev fp32 [3,HW]; angles_out_dev fp32 [HW] or NULL: degrees, NaN where ||gt|| == 0.
+ * out_host[9] = {n_valid, mean, median, rmse, %<5, %<7.5, %<11.25, %<22.5, %<30} (NaN metrics when n_valid == 0). */
+int mgb_eval_normals(const float* pred_dev, const float* gt_dev, int64_t HW, float* angles_out_dev, void* ws_dev,
+                     double* out_host, void* stream);
+/* compute_iid_metric(metric_name="psnr") (src/util/metric.py:263-338 as script/iid/eval.py:182-213 calls it) with ONE
+ * synchronisation. pred_dev, gt_dev fp32 [3,HW]; mask_dev uint8 [3,HW] or NULL. transform: 0 none, 1 srgb2linear
+ * (x ** 2.2), 2 linear2srgb (x ** (1 / 2.2)), applied to both first. align = 1 (shading, residual): least-squares scale
+ * (compute_alignment_scale) and quantile_map, whose 0.9 quantile is an exact order statistic on the device.
+ * out_host[5] = {psnr, lstsq_scale, quantile, quantile_scale, n} (the three alignment values NaN when align = 0). */
+int mgb_eval_iid(const float* pred_dev, const float* gt_dev, const uint8_t* mask_dev, int64_t HW, int32_t align,
+                 int32_t transform, void* ws_dev, double* out_host, void* stream);
 
 /* ---- capacity ------------------------------------------------------------------------------- */
 /* Bytes of the activation arena the handle holds for images of H x W with B members per batch. */

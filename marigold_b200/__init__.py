@@ -6,7 +6,7 @@ Importing the package does not load the CUDA library; the first Engine()/ensembl
 fails loudly if it is unavailable (no CPU fallback)."""
 from .engine import Engine, EngineConfig  # noqa: F401
 from .ensemble import ensemble_depth, ensemble_iid, ensemble_normals  # noqa: F401
-from .evaluation import align_depth_least_square, evaluate_depth  # noqa: F401
+from .evaluation import align_depth_least_square, evaluate_depth, evaluate_iid, evaluate_normals  # noqa: F401
 from .iid import IIDEntry, MarigoldIIDOutput  # noqa: F401
 from .pipeline import (  # noqa: F401
     MarigoldDepthOutput,

@@ -65,6 +65,8 @@ SIGNATURES = {
     "mgb_colorize": (_i32, [_vp, _i64, _f32, _f32, _vp, _vp, _vp]),
     "mgb_eval_ws_bytes": (C.c_size_t, []),
     "mgb_eval_depth": (_i32, [_vp, _vp, _vp, _i64, _i32, _f32, _f32, _vp, _vp, _vp, _vp]),
+    "mgb_eval_normals": (_i32, [_vp, _vp, _i64, _vp, _vp, _vp, _vp]),
+    "mgb_eval_iid": (_i32, [_vp, _vp, _vp, _i64, _i32, _i32, _vp, _vp, _vp]),
     "mgb_workspace_bytes": (C.c_size_t, [_vp, _i32, _i32, _i32]),
     "mgb_launch_count": (_i64, []),
     "mgb_op_linear": (_i32, [_vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp]),

@@ -147,18 +147,49 @@ int mgb_colorize(const float* depth, int64_t HW, float dmin, float dmax, const u
 
 size_t mgb_eval_ws_bytes(void) { return eval_ws_bytes() + 16 * sizeof(double); }
 
-int mgb_eval_depth(const float* pred, const float* gt, const uint8_t* mask, int64_t HW, int32_t least_squares, float dmin,
+// copies n result doubles to the host and synchronises (the one synchronisation of each mgb_eval_* call)
+static int eval_fetch(const char* what, double* out_host, const double* out_dev, int n, cudaStream_t s) {
+  cudaError_t e = cudaMemcpyAsync(out_host, out_dev, n * sizeof(double), cudaMemcpyDeviceToHost, s);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+  if (e != cudaSuccess) { set_error("%s: %s", what, cudaGetErrorString(e)); return MGB_ERR_CUDA; }
+  return MGB_OK;
+}
+
+int mgb_eval_depth(const float* pred, const float* gt, const uint8_t* mask, int64_t HW, int32_t alignment, float dmin,
                    float dmax, float* aligned_out, void* ws, double* out_host, void* stream) {
-  if (!pred || !gt || !ws || !out_host || HW <= 0) { set_error("mgb_eval_depth: bad argument"); return MGB_ERR_INVALID; }
+  if (!pred || !gt || !ws || !out_host || HW <= 0 || alignment < 0 || alignment > 2) {
+    set_error("mgb_eval_depth: bad argument"); return MGB_ERR_INVALID;
+  }
   double* out_dev = reinterpret_cast<double*>(static_cast<char*>(ws) + eval_ws_bytes());
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  int rc = launch_eval_depth(pred, gt, mask, HW, least_squares, dmin, dmax, aligned_out, ws, out_dev, s);
+  int rc = launch_eval_depth(pred, gt, mask, HW, alignment, dmin, dmax, aligned_out, ws, out_dev, s);
   if (rc) return rc;
   count_launch(4);
-  cudaError_t e = cudaMemcpyAsync(out_host, out_dev, 13 * sizeof(double), cudaMemcpyDeviceToHost, s);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-  if (e != cudaSuccess) { set_error("mgb_eval_depth: %s", cudaGetErrorString(e)); return MGB_ERR_CUDA; }
-  return MGB_OK;
+  return eval_fetch("mgb_eval_depth", out_host, out_dev, 13, s);
+}
+
+int mgb_eval_normals(const float* pred, const float* gt, int64_t HW, float* angles_out, void* ws, double* out_host,
+                     void* stream) {
+  if (!pred || !gt || !ws || !out_host || HW <= 0) { set_error("mgb_eval_normals: bad argument"); return MGB_ERR_INVALID; }
+  double* out_dev = reinterpret_cast<double*>(static_cast<char*>(ws) + eval_ws_bytes());
+  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+  int rc = launch_eval_normals(pred, gt, HW, angles_out, ws, out_dev, s);
+  if (rc) return rc;
+  count_launch(11);                                  // memset, sums, count, 3 x (histogram + pick), above, final
+  return eval_fetch("mgb_eval_normals", out_host, out_dev, 9, s);
+}
+
+int mgb_eval_iid(const float* pred, const float* gt, const uint8_t* mask, int64_t HW, int32_t align, int32_t transform,
+                 void* ws, double* out_host, void* stream) {
+  if (!pred || !gt || !ws || !out_host || HW <= 0 || transform < 0 || transform > 2) {
+    set_error("mgb_eval_iid: bad argument"); return MGB_ERR_INVALID;
+  }
+  double* out_dev = reinterpret_cast<double*>(static_cast<char*>(ws) + eval_ws_bytes());
+  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+  int rc = launch_eval_iid(pred, gt, mask, HW, align != 0, transform, ws, out_dev, s);
+  if (rc) return rc;
+  count_launch(align ? 12 : 2);                      // [memset, sums, solve, 7 selection, quantile], psnr sums, final
+  return eval_fetch("mgb_eval_iid", out_host, out_dev, 5, s);
 }
 
 int mgb_op_space_to_depth(const float* x, void* y, int32_t NB, int32_t H, int32_t W, int32_t C, void* stream) {

@@ -173,8 +173,16 @@ int launch_resize(const void* src, int src_is_u8, int NC, int H, int W, float* d
 int launch_colorize(const float* depth, long long HW, float dmin, float dmax, const uint8_t* lut, uint8_t* out,
                     cudaStream_t stream);
 size_t eval_ws_bytes();
-int launch_eval_depth(const float* pred, const float* gt, const uint8_t* mask, long long HW, int do_align, float dmin, float dmax,
+// alignment 0 none, 1 least squares in depth, 2 least squares in disparity; out_dev: 13 doubles
+int launch_eval_depth(const float* pred, const float* gt, const uint8_t* mask, long long HW, int alignment, float dmin, float dmax,
                       float* aligned_out, void* ws, double* out_dev, cudaStream_t stream);
+// pred, gt [3, HW]; angles_out [HW] or null; out_dev: 9 doubles {n_valid, mean, median, rmse, sub5 .. sub30}
+int launch_eval_normals(const float* pred, const float* gt, long long HW, float* angles_out, void* ws, double* out_dev,
+                        cudaStream_t stream);
+// pred, gt, mask (or null) [3, HW]; transform 0 / 1 / 2 (none, ** 2.2, ** (1 / 2.2)); out_dev: 5 doubles
+// {psnr, lstsq_scale, quantile, quantile_scale, n}
+int launch_eval_iid(const float* pred, const float* gt, const uint8_t* mask, long long HW, int align, int transform, void* ws,
+                    double* out_dev, cudaStream_t stream);
 
 // ---------------------------------------------------------------------------------------------
 // Ensemble kernels (ensemble.cu)
